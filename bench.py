@@ -40,7 +40,14 @@ def parse_args():
     ap.add_argument("--no-verify", action="store_true", help="skip the oracle digest check of the produced stream (outside the timed region)")
     ap.add_argument("--no-config5", action="store_true", help="N > 1: skip the 8 GiB-per-GPU encode-only / gather-inclusive extra")
     ap.add_argument("--config5-bytes", type=int, default=8 * GiB)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's output (stream size and a seeded sample of the stream) to DIR/*.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
+    return args
 
 
 def measured_peaks():
@@ -187,6 +194,31 @@ def verify_against_oracle(dev, world, rank, n, d_out, out_bytes, dist, torch, sy
     return res
 
 
+DUMP_WINDOWS, DUMP_WINDOW_BYTES = 1024, 8192     # 8 MiB of stream over all ranks, 32 MiB as float32
+
+
+def dump_outputs(dirname, suffix, d_out, out_bytes, windows, d_flags=None):
+    """What a caller of the timed path receives: the encoded size, the stream and (sharded) the flags, as float arrays. A stream
+    longer than `windows` x DUMP_WINDOW_BYTES is sampled in windows at offsets drawn from a fixed seed, so that two builds run
+    with the same arguments are compared on the same bytes."""
+    import numpy as np
+    import torch
+    os.makedirs(dirname, exist_ok=True)
+    if out_bytes <= windows * DUMP_WINDOW_BYTES:
+        offs = np.zeros(1, dtype=np.int64)
+        sample = d_out[:out_bytes][None]
+    else:
+        offs = np.sort(np.random.default_rng(0).integers(0, out_bytes - DUMP_WINDOW_BYTES + 1, size=windows))
+        idx = torch.from_numpy(offs).to(d_out.device)[:, None] + torch.arange(DUMP_WINDOW_BYTES, device=d_out.device)
+        sample = d_out[idx]
+    arrays = {"stream_size": np.array([out_bytes], dtype=np.float64), "stream_sample": sample.float().cpu().numpy(),
+              "stream_sample_offsets": offs.astype(np.float64)}
+    if d_flags is not None:
+        arrays["flags"] = d_flags.double().cpu().numpy()
+    for name, a in arrays.items():
+        np.save(os.path.join(dirname, name + suffix + ".npy"), a)
+
+
 def cpu_rate(alg, op, sample, reps=3):
     """oracle port on one host core: input GB/s (uncompressed bytes / time, benches/density.rs:29,48)"""
     import numpy as np
@@ -290,6 +322,9 @@ def run_ours(args):
     stage_ms = [float(x) for x in t[1:].tolist()]
     ms_per_step = total_ms / args.steps
     value = world * n / (ms_per_step * 1e-3) / 1e9
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, f"_rank{rank}" if world > 1 else "", d_out, int(d_size.item()), DUMP_WINDOWS // world,
+                     d_flags if world > 1 else None)
 
     # ---- parity, outside the timed region: the stream(s) just produced against ONE oracle call over the whole input --------------
     parity = None
@@ -413,9 +448,8 @@ def run_ours(args):
             del d_k, d_ok
         # config 1: Chameleon round trip on Silesia/dickens through the reference symbols (latency-bound on a GPU; reported, not optimised)
         dk = None
-        # the file: the reference's convention (benches/utils.rs:6-17): $FILE, else benches/data/dickens.txt (a copy travels in oracle/_ref)
-        cands = [(os.path.join(ROOT, "oracle", "_ref", "dickens.txt"), "benches/data/dickens.txt (10,192,446 B)"),
-                 (os.path.join(ROOT, "tests", "golden", "dickens_200k.bin"), "first 200,000 B of dickens (tests/golden)")]
+        # the file: $FILE as in the reference's benches (utils.rs:6-17), else the first 200,003 B of dickens kept in the tree
+        cands = [(os.path.join(ROOT, "tests", "golden", "dickens_200k.bin"), "first 200,003 B of dickens (tests/golden)")]
         if os.environ.get("FILE"):
             cands.insert(0, (os.environ["FILE"], "FILE=" + os.environ["FILE"]))
         for cand, label in cands:

@@ -50,10 +50,9 @@ def golden_inputs(dickens200k):
         "zeros_1m": np.zeros(1 << 20, dtype=np.uint8),
         "splitmix_1m_seed1": splitmix_bytes(1 << 20, 1),
         "mixed_280004": np.concatenate([d[:100000], splitmix_bytes(50001, 7), np.zeros(30000, np.uint8), d[100000:200003]]),
+        # stands in for the whole 10 MB file, whose digests stay in golden.json for test_published_dickens_ratios
+        "dickens_sample_256k": np.fromfile(os.path.join(GOLDEN_DIR, "dickens_sample_256k.bin"), dtype=np.uint8),
     }
-    ref = "/root/reference/benches/data/dickens.txt"
-    if os.path.exists(ref):  # authoring container only; never on the GPU box
-        cases["dickens_full"] = np.fromfile(ref, dtype=np.uint8)
     return cases
 
 

@@ -1,9 +1,9 @@
-"""Regenerates tests/golden/*.  Run in the authoring container (needs /root/reference for the dickens corpus):
+"""Regenerates tests/golden/* from the Silesia corpus file `dickens` (10,192,446 bytes):
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py path/to/dickens
 
 The expected outputs are produced by the oracle (oracle/density_oracle.c), which is itself pinned on the reference's
-known-answer vectors (/root/reference/src/lib.rs:19,28,50,72). The reference is Rust and cannot be built in this image,
+known-answer vectors (the reference's src/lib.rs:19,28,50,72). The reference is Rust and this project does not build it,
 so these fixtures are "oracle outputs cross-checked against the reference's published facts":
   * the three KATs (exact bytes),
   * dickens compressed sizes 5,827,114 / 5,480,246 / 5,183,816 <=> ratios 1.749x/1.860x/1.966x (benchmark.log:17,22,27),
@@ -20,7 +20,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(HERE, "..", ".."))
 import oracle  # noqa: E402
 
-DICKENS = "/root/reference/benches/data/dickens.txt"
+SAMPLE_PIECES, SAMPLE_PIECE_BYTES = 16, 16384
 
 
 def splitmix_bytes(n, seed):
@@ -36,9 +36,17 @@ def splitmix_bytes(n, seed):
     return out.view(np.uint8)[:n].copy()
 
 
-def main():
-    d = np.frombuffer(open(DICKENS, "rb").read(), dtype=np.uint8)
+def dickens_sample(d):
+    """16 KiB pieces at 16 evenly spaced offsets of the whole file: the full file is too large to keep in the tree."""
+    step = d.size // SAMPLE_PIECES
+    return np.concatenate([d[k * step:k * step + SAMPLE_PIECE_BYTES] for k in range(SAMPLE_PIECES)])
+
+
+def main(path):
+    d = np.frombuffer(open(path, "rb").read(), dtype=np.uint8)
     d[:200003].tofile(os.path.join(HERE, "dickens_200k.bin"))
+    sample = dickens_sample(d)
+    sample.tofile(os.path.join(HERE, "dickens_sample_256k.bin"))
     cases = {
         "kat": np.frombuffer(b"test" * 31 + b"t", dtype=np.uint8),
         "dickens_65539": d[:65539],
@@ -46,6 +54,7 @@ def main():
         "splitmix_1m_seed1": splitmix_bytes(1 << 20, 1),
         "mixed_280004": np.concatenate([d[:100000], splitmix_bytes(50001, 7), np.zeros(30000, np.uint8), d[100000:200003]]),
         "dickens_full": d,
+        "dickens_sample_256k": sample,
     }
     gold = {}
     for name, data in cases.items():
@@ -63,4 +72,4 @@ def main():
 
 
 if __name__ == "__main__":
-    main()
+    main(sys.argv[1])

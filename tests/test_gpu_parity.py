@@ -55,8 +55,6 @@ def test_reference_kats_through_c_abi(codecs, alg, golden):
 def test_golden_fixtures_encode_decode(codecs, alg, golden, golden_inputs):
     C = codecs[alg]
     for name, data in golden_inputs.items():
-        if name == "dickens_full":
-            continue
         enc = gpu_encode(C, data)
         e = golden[name]["alg"][alg]
         assert (enc.size, sha256(enc)) == (e["size"], e["sha256"]), (alg, name)
